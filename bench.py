@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's engine, N GPUs of one node
     python bench.py --impl reference --steps K --warmup W    # the reference's own AgentPPO on the host cores (oracle/_ref)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + one step's outputs from the seeded start, as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8(d)): AgentPPO on Pendulum-v1, 65 536 envs PER GPU
 (env-sharded, weak scaling), horizon 128, 2x64 GELU MLP actor + critic, Config defaults batch_size=128,
@@ -30,6 +31,8 @@ UNIT = "env-steps/s"
 FLOP_PER_ENV_STEP = 17408          # actor fwd 8704 + critic fwd 8704 (SURVEY 8(d))
 HBM_BYTES_PER_ENV_STEP = 30        # 26 B trajectory + 4 B value written by the fused rollout kernel
 NCU_DRAM_BYTES_PER_LAUNCH = 198.11e6  # measured once with ncu (2.22 MB read + 195.89 MB written), profiles/r02_v2_rollout_ts_metrics.txt
+DUMP_ENVS = 4096                   # env columns --dump-outputs keeps of the rollout buffer: 17 MB in all at horizon 128
+BUFFER_NAMES = ("states", "actions", "logprobs", "rewards", "undones", "unmasks")
 
 
 def workload_config(n_gpus, num_envs=None):
@@ -152,6 +155,26 @@ def calibrate_threads(time_fn, num_envs=NUM_ENVS, cache=os.path.join("/tmp", "b2
     return best, scores
 
 
+def dump_outputs(out_dir, buffer, losses, agent):
+    """Write what one cycle handed its caller as float32 ``out_dir/<name>.npy``, so that two builds run with the same arguments
+    can be compared output for output: the six buffer tensors as the caller holds them after ``update_net_device`` (which
+    rewrites rewards / undones in place, as the reference does) and ``last_state``, on a fixed, seeded sample of env columns;
+    the three losses; the actor and critic parameters after the update."""
+    import numpy as np
+    import torch as th
+    os.makedirs(out_dir, exist_ok=True)
+    n = buffer[0].shape[1]
+    cols = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_ENVS), replace=False))
+    idx = th.from_numpy(cols).to(buffer[0].device)
+    arrays = {name: t.index_select(1, idx) for name, t in zip(BUFFER_NAMES, buffer)}
+    arrays["last_state"] = agent.last_state.index_select(0, idx)
+    arrays["losses"] = losses
+    for prefix, module in (("act", agent.act), ("cri", agent.cri)):
+        arrays.update({f"{prefix}.{k}": v for k, v in module.state_dict().items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def run_reference(args):
     """The reference's own CPU implementation of the path (see cpu_backend) on the host cores, same config / metric;
     rank 0 only.  Each step is a full cycle at 65 536 envs unless K + W such cycles would not fit in ~3 minutes; then
@@ -205,15 +228,21 @@ def run_engine(args):
                 'if_discrete': False}
     cfg = Config(AgentPPO, PendulumVecEnv, env_args)
     cfg.net_dims, cfg.batch_size, cfg.repeat_times, cfg.random_seed = NET_DIMS, BATCH_SIZE, REPEAT_TIMES, 0
-    th.manual_seed(0)  # identical initial parameters on every rank
-    agent = AgentPPO(NET_DIMS, 3, 1, gpu_id=local_rank, args=cfg)
-    if world > 1:
-        agent.enable_data_parallel()
-        agent.sharded_mode = args.sharded_mode
-    env = PendulumVecEnv(num_envs=n_envs, gpu_id=local_rank, max_step=200, seed=rank)
-    agent.last_state = env.reset()[0]
-    # stagger episode phases like a long-running job (otherwise every env truncates at the same step)
-    env.cur_step[:] = th.randint(0, 200, (n_envs,), device=dev, dtype=th.int32)
+
+    def make_agent_env():
+        """Agent and env from fixed seeds: the same inputs on every run with the same arguments."""
+        th.manual_seed(0)  # identical initial parameters on every rank
+        agent = AgentPPO(NET_DIMS, 3, 1, gpu_id=local_rank, args=cfg)
+        if world > 1:
+            agent.enable_data_parallel()
+            agent.sharded_mode = args.sharded_mode
+        env = PendulumVecEnv(num_envs=n_envs, gpu_id=local_rank, max_step=200, seed=rank)
+        agent.last_state = env.reset()[0]
+        # stagger episode phases like a long-running job (otherwise every env truncates at the same step)
+        env.cur_step[:] = th.randint(0, 200, (n_envs,), device=dev, dtype=th.int32)
+        return agent, env
+
+    agent, env = make_agent_env()
 
     def barrier():
         if world > 1:
@@ -300,6 +329,17 @@ def run_engine(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     e2e_ms = float(t.item())
 
+    if args.dump_outputs:
+        # The update's floating-point sums are not bit-reproducible and Pendulum amplifies the last bits over a few cycles, so
+        # the state after the timed steps differs from run to run.  The step that is written out is one step of the timed
+        # path from the seeded initial state instead: identical inputs on every run, comparable outputs across builds.
+        dump_agent, dump_env = make_agent_env()
+        buffer = dump_agent.explore_env(dump_env, HORIZON)
+        losses = dump_agent.update_net_device(list(buffer))
+        barrier()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, buffer, losses, dump_agent)
+
     env_steps = n_envs * HORIZON * args.steps * world
     value = env_steps / (elapsed_ms * 1e-3)
     peaks = measured_peaks()
@@ -363,7 +403,12 @@ def main():
     ap.add_argument("--total-envs", type=int, default=None, help="strong-scaling study: this many envs in total, split over the GPUs")
     ap.add_argument("--sharded-mode", default="auto", choices=["auto", "peer", "peer_allreduce", "gather", "allreduce"],
                     help="N > 1: how the env shards' gradients meet (auto = in-kernel peer-memory exchange when available)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, run one more step of the timed path from the seeded initial state and write what "
+                         "it computed (buffer sample, losses, parameters) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

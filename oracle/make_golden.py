@@ -842,3 +842,44 @@ def main_tc_shapes():
 
 if __name__ == "__main__" and os.environ.get("GOLDEN_ONLY", "") in ("", "tcshapes"):
     main_tc_shapes()
+
+
+# --------------------------------------------------------------------------- evaluator rollout (SURVEY section 8 row f4)
+# (num_envs, max_step, seed and rows of the injected reset noise)
+EVALUATOR_CASES = ((24, 30, 3, 64), (24, 30, 11, 32), (1344, 40, 11, 42))
+
+
+def evaluator_actor():
+    """The actor of tests/test_evaluator.py: ActorPPO 2x64 from th.manual_seed(5), biases perturbed."""
+    from elegantrl_b200.agents.nets import ActorPPO
+    th.manual_seed(5)
+    actor = ActorPPO([64, 64], 3, 1)
+    with th.no_grad():
+        for layer in actor.net:
+            if hasattr(layer, "bias"):
+                layer.bias += 0.1 * th.randn_like(layer.bias)
+    return actor
+
+
+def main_evaluator():
+    """The reference's ``get_cumulative_rewards_and_step_from_vec_env`` (``elegantrl/train/evaluator.py:200-238``) on the
+    CPU torch Pendulum vec env with reset noise of ``th.rand((rows, n, 2))`` from a seeded generator: the (return, steps)
+    list of every case, in the reference's order, and the actor's parameters."""
+    from elegantrl.train.evaluator import get_cumulative_rewards_and_step_from_vec_env as ref_fn
+    os.makedirs(OUT_DIR, exist_ok=True)
+    th.set_num_threads(1)
+    actor = evaluator_actor()
+    out = {f"actor.{k}": v.numpy().copy() for k, v in actor.state_dict().items()}
+    for n, max_step, seed, rows in EVALUATOR_CASES:
+        env = PendulumVecEnv(num_envs=n, gpu_id=-1, max_step=max_step)
+        env.inject_reset_noise(th.rand((rows, n, 2), generator=th.Generator().manual_seed(seed)))
+        with th.no_grad():
+            got = ref_fn(env, actor)
+        out[f"n{n}_t{max_step}_s{seed}.returns"] = np.array([r for r, _ in got], dtype=np.float32)
+        out[f"n{n}_t{max_step}_s{seed}.steps"] = np.array([s for _, s in got], dtype=np.int64)
+    np.savez_compressed(os.path.join(OUT_DIR, "evaluator_pendulum.npz"), **out)
+    print(f"| wrote evaluator_pendulum.npz  ({len(out)} arrays)")
+
+
+if __name__ == "__main__" and os.environ.get("GOLDEN_ONLY", "") in ("", "evaluator"):
+    main_evaluator()

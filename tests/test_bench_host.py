@@ -54,3 +54,35 @@ def test_both_arms_describe_the_same_workload():
         assert bench.workload_config(n) == bench.workload_config(n, bench.NUM_ENVS)
     src = open(bench.__file__).read()
     assert '"config": workload_config(args.gpus)' in src and '"config": workload_config(world, n_envs)' in src
+
+
+def test_dump_outputs_writes_a_seeded_float32_sample(tmp_path):
+    """--dump-outputs: one float32 .npy per output; the same env columns on every call; the full-size buffer stays far below
+    64 MB."""
+    import numpy as np
+    import torch as th
+    from elegantrl_b200.agents.nets import ActorPPO, CriticPPO
+    h, n = 128, bench.NUM_ENVS
+    g = th.Generator().manual_seed(0)
+    buffer = [th.rand((h, n, 3), generator=g), th.rand((h, n, 1), generator=g), th.rand((h, n), generator=g),
+              th.rand((h, n), generator=g), th.ones((h, n), dtype=th.bool), th.rand((h, n), generator=g) > 0.01]
+    agent = type("Agent", (), dict(last_state=th.rand((n, 3), generator=g), act=ActorPPO([64, 64], 3, 1),
+                                   cri=CriticPPO([64, 64], 3, 1)))()
+    buffer[0][..., 0] = th.arange(n, dtype=th.float32)      # the env index, to see which columns were kept
+    losses = th.tensor([0.5, -0.25, 1.4])
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), buffer, losses, agent)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == sorted(p.name for p in (tmp_path / "b").iterdir())
+    assert {f"{k}.npy" for k in bench.BUFFER_NAMES + ("last_state", "losses", "act.net.0.weight", "cri.net.4.bias")} <= set(files)
+    total = 0
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b), f
+        total += a.nbytes
+    assert total <= 64 << 20
+    states = np.load(tmp_path / "a" / "states.npy")
+    assert states.shape == (h, bench.DUMP_ENVS, 3)
+    cols = states[0, :, 0].astype(np.int64)
+    assert len(np.unique(cols)) == bench.DUMP_ENVS and np.array_equal(states, buffer[0].numpy()[:, cols])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "losses.npy"), losses.numpy())

@@ -1,15 +1,12 @@
 """SURVEY section 8 row f4 (evaluator rollout): ``elegantrl_b200.train.evaluator`` against the reference's own
-``get_cumulative_rewards_and_step_from_vec_env`` (``elegantrl/train/evaluator.py:200-238``, imported from the byte-for-byte
-copy in oracle/_ref)."""
-import os
-import sys
-
+``get_cumulative_rewards_and_step_from_vec_env`` (``elegantrl/train/evaluator.py:200-238``): the (return, steps) lists it
+produced for the same actor and injected reset noise are stored in ``tests/golden/evaluator_pendulum.npz``
+(``oracle/make_golden.py::main_evaluator``)."""
 import numpy as np
 import pytest
 import torch as th
 
-REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = os.path.join(REPO, "oracle", "_ref")
+from tests import golden_utils as gu
 
 
 def _reference_segmentation(returns, dones):
@@ -36,40 +33,30 @@ def test_episode_segmentation_matches_the_reference_loop(t_len, n, p):
     np.testing.assert_allclose([r for r, _ in got], [r for r, _ in want], rtol=1e-5, atol=1e-5)
 
 
-def _reference_function():
-    if not os.path.isdir(os.path.join(REF, "elegantrl")):
-        pytest.skip("oracle/_ref is absent: run `python oracle/make_ref.py` in the build container")
-    sys.path.insert(0, REF)
-    try:
-        from elegantrl.train.evaluator import get_cumulative_rewards_and_step_from_vec_env as ref_fn
-    finally:
-        sys.path.remove(REF)
-    return ref_fn
+def _reference_result(n, max_step, seed):
+    """What the reference function returned on the CPU env with ``n`` envs, ``max_step`` and reset-noise seed ``seed``."""
+    g = gu.load("evaluator_pendulum")
+    return list(zip(g[f"n{n}_t{max_step}_s{seed}.returns"].tolist(), g[f"n{n}_t{max_step}_s{seed}.steps"].tolist()))
 
 
 def _actor(device):
+    """ActorPPO 2x64 with the parameters the golden was minted with (seeded init, perturbed biases)."""
     from elegantrl_b200.agents.nets import ActorPPO
-    th.manual_seed(5)
-    actor = ActorPPO([64, 64], 3, 1)          # built on the CPU (one RNG stream), then moved: identical weights on every device
-    with th.no_grad():
-        for layer in actor.net:
-            if hasattr(layer, "bias"):
-                layer.bias += 0.1 * th.randn_like(layer.bias)
+    g = gu.load("evaluator_pendulum")
+    actor = ActorPPO([64, 64], 3, 1)
+    actor.load_state_dict({k[len("actor."):]: th.from_numpy(v) for k, v in g.items() if k.startswith("actor.")})
     return actor.to(device)
 
 
 def test_generic_path_equals_reference_function_on_cpu():
     from elegantrl_b200.envs import PendulumVecEnv
     from elegantrl_b200.train.evaluator import get_cumulative_rewards_and_step_from_vec_env
-    ref_fn = _reference_function()
     actor = _actor("cpu")
     noise = th.rand((64, 24, 2), generator=th.Generator().manual_seed(3))
-    out = []
-    for fn in (ref_fn, get_cumulative_rewards_and_step_from_vec_env):
-        env = PendulumVecEnv(num_envs=24, gpu_id=-1, max_step=30)
-        env.inject_reset_noise(noise)
-        with th.no_grad():
-            out.append(fn(env, actor))
+    env = PendulumVecEnv(num_envs=24, gpu_id=-1, max_step=30)
+    env.inject_reset_noise(noise)
+    with th.no_grad():
+        out = [_reference_result(24, 30, 3), get_cumulative_rewards_and_step_from_vec_env(env, actor)]
     assert [s for _, s in out[0]] == [s for _, s in out[1]] == [30] * 24
     np.testing.assert_allclose([r for r, _ in out[1]], [r for r, _ in out[0]], rtol=1e-5, atol=1e-5)
 
@@ -81,14 +68,9 @@ def test_fused_evaluation_rollout_equals_reference_function(n, max_step):
     (CPU) with the torch actor, same injected reset noise."""
     from elegantrl_b200.envs import PendulumVecEnv
     from elegantrl_b200.train import evaluator as ev
-    ref_fn = _reference_function()
-    actor_cpu = _actor("cpu")
     actor_gpu = _actor("cuda:0")
     noise = th.rand((max_step + 2, n, 2), generator=th.Generator().manual_seed(11))
-    env_cpu = PendulumVecEnv(num_envs=n, gpu_id=-1, max_step=max_step)
-    env_cpu.inject_reset_noise(noise)
-    with th.no_grad():
-        want = ref_fn(env_cpu, actor_cpu)
+    want = _reference_result(n, max_step, 11)
     env_gpu = PendulumVecEnv(num_envs=n, gpu_id=0, max_step=max_step)
     env_gpu.inject_reset_noise(noise)
     assert ev._fused_pendulum_ok(env_gpu, actor_gpu)
